@@ -2,7 +2,7 @@
 """bench.py -- BA solver iterations/s on synthetic sliding windows (BASELINE.json metric).
 
     python bench.py --gpus N --steps K --warmup W [--batch B] [--iters I] [--impl reference]
-                    [--cams mono|stereo|quad] [--rho-sweep] [--swarm-agents A --swarms S]
+                    [--cams mono|stereo|quad] [--rho-sweep] [--swarm-agents A --swarms S] [--dump-outputs DIR]
 
 A "step" = one solve of `iters` trust-region iterations (fixed schedule, convergence exits off so the
 work per step is constant) on every window of the batch.  An iteration = one trust-region step attempt:
@@ -17,6 +17,9 @@ carries (a) `latency_b1`: one window through the reference-style reset -> add ->
 handle on one GPU (ADMM, consensus reduced on the device) next to the CPU path with 4 threads and with all cores.
 N>1 (configs[2], [3]): N-drone swarms, one agent per GPU, ADMM with the NCCL consensus exchange per sub-step; every rank
 solves its agent's window of B swarms.  `--cams quad --rho-sweep` is config 4's quadcam / rho sweep mode.
+`--dump-outputs DIR` writes what the last timed step handed back (see dump_outputs); the inputs are seeded, so two builds run
+with the same arguments can be compared output for output.  Compare with a tolerance: the device's reductions are not
+summed in a fixed order, and two runs of one build on a B200 (1000 W) differed by up to 1e-9 relative in the solved state.
 """
 import argparse
 import contextlib
@@ -37,6 +40,8 @@ from d2slam_b200 import abi, synth  # noqa: E402
 
 OBS_BYTES = 176                      # SURVEY.md 8d: 20 f64 constants + 4 i32 ids
 IMU_BYTES = 3736 + 3720
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_FILES = 8                       # pose, extrinsic, speed_bias, inv_depth, td, initial_cost, final_cost, window
 RHO_SWEEP = [(1.0, 1.0), (10.0, 10.0), (100.0, 100.0), (1000.0, 1000.0), (10.0, 1000.0)]   # rho_T = rho_theta and one rho_T != rho_theta (consenus_factor.cpp:15-16)
 
 
@@ -180,6 +185,27 @@ def d2h_bytes(probs):
     return int(sum(p["poses"].nbytes + p["sb"].nbytes + p["inv_dep"].nbytes for p in probs))
 
 
+def dump_outputs(directory, get_blocks, probs, reps, suffix=""):
+    """What the timed solve hands back to its caller, per window in batch order: the solved blocks (get_blocks(window, kind, ids))
+    and the report's costs, concatenated over windows as float64 `<name><suffix>.npy`.  A batch whose outputs exceed 64 MB is
+    reduced to a fixed, seeded sample of windows; `window.npy` lists the windows written."""
+    per_window = [8 * (7 * (len(p["frame_ids"]) + len(p["cam_ids"])) + 9 * len(p["sb_ids"]) + len(p["lm_ids"]) + 4) for p in probs]
+    budget = DUMP_LIMIT_BYTES - DUMP_FILES * 128      # an .npy header takes at most 128 bytes here (short names, 1-2 dims)
+    keep = np.arange(len(probs))
+    if sum(per_window) > budget:
+        keep = np.sort(np.random.default_rng(0).permutation(len(probs))[: budget // max(per_window)])
+    blocks = {"pose": (abi.POSE, "frame_ids"), "extrinsic": (abi.EXTRINSIC, "cam_ids"), "speed_bias": (abi.SPEED_BIAS, "sb_ids"), "inv_depth": (abi.LANDMARK, "lm_ids")}
+    out = {name: np.concatenate([get_blocks(int(i), kind, probs[i][ids]) for i in keep]) for name, (kind, ids) in blocks.items()}
+    out["inv_depth"] = out["inv_depth"][:, 0]
+    out["td"] = np.array([get_blocks(int(i), abi.TD, np.zeros(1, np.int64))[0, 0] for i in keep])
+    out["initial_cost"] = np.array([reps[i].initial_cost for i in keep])
+    out["final_cost"] = np.array([reps[i].final_cost for i in keep])
+    out["window"] = keep.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, f"{name}{suffix}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def oracle_of(p, **cfg):
     from oracle import orc
     o = orc.Oracle(**cfg); p.load(o)
@@ -226,6 +252,7 @@ def run_reference(args, rank, world):
         probs = make_batch(n_units, 1000, cams=args.cams)
         oras = [oracle_of(p, max_num_iterations=iters) for p in probs]
         run = lambda m, nt=cores: orc.solve_many(oras[:m], nt, fixed_iters=iters)
+        units = lambda m: list(zip(oras[:m], probs[:m]))
         workload = f"W1 single-drone 11-frame/300-landmark windows ({args.cams}), {iters} trust-region iterations per solve"
         unit = "windows"
 
@@ -240,6 +267,7 @@ def run_reference(args, rank, world):
         swarms = [[oracle_of(p, max_num_iterations=iters, consensus_max_steps=args.admm_steps) for p in base[i % distinct]] for i in range(min(n_units, 4 * distinct))]
         n_units = len(swarms)
         run = lambda m, nt=cores: orc.admm_many(swarms[:m], nt, fixed_mode=True)
+        units = lambda m: [(o, p) for i, sw in enumerate(swarms[:m]) for o, p in zip(sw, base[i % distinct])]
         workload = (f"{n_agents}-drone swarm ({args.cams}), 11-frame/300-landmark windows + {(n_agents - 1) * 11} remote poses per agent, "
                     f"ADMM {args.admm_steps} sub-steps x {max(1, iters // args.admm_steps)} iterations")
         unit = "swarms"
@@ -264,6 +292,9 @@ def run_reference(args, rank, world):
         its = sum(r.total_iterations for r in reps)
         if s >= args.warmup:
             vals.append((its / dt, dt))
+        if args.dump_outputs and s == args.warmup + args.steps - 1:
+            u = units(m_units)
+            dump_outputs(args.dump_outputs, lambda i, kind, ids: u[i][0].get_blocks(kind, ids), [p for _, p in u], reps)
         if s == 0 and dt * (args.warmup + args.steps) > budget_s:
             m_units = max(min(cores, n_units), int(n_units * budget_s / (dt * (args.warmup + args.steps))))
             note = f"; reduced to {m_units} {unit} per step after the first one to keep the run within {budget_s:.0f} s"
@@ -287,13 +318,14 @@ def run_reference(args, rank, world):
 # ------------------------------------------------------------------------------------------------ our arm: helpers
 def timed_solves(solver, probs, iters, steps, warmup, barrier=None, step_barrier=None):
     """Device-resident throughput: problem already in HBM, only the (small) state is restored per step.
-    -> (device seconds summed over steps [CUDA events on the solver stream], wall seconds)"""
+    -> (device seconds summed over steps [CUDA events on the solver stream], wall seconds, reports of the last step)"""
     for _ in range(warmup):
         reset_state(solver, probs); solver.solve_fixed(iters)
     if barrier:
         barrier()
     t0 = time.perf_counter()
     dev_ms = 0.0
+    reps = None
     for _ in range(steps):
         reset_state(solver, probs)
         if step_barrier:
@@ -302,7 +334,7 @@ def timed_solves(solver, probs, iters, steps, warmup, barrier=None, step_barrier
         dev_ms += reps[0].total_time * 1e3
     if barrier:
         barrier()
-    return dev_ms * 1e-3, time.perf_counter() - t0
+    return dev_ms * 1e-3, time.perf_counter() - t0, reps
 
 
 def latency_b1(local_rank, iters, cams):
@@ -362,7 +394,7 @@ def swarm_one_gpu(args, local_rank, n_agents, n_swarms, iters, steps, warmup, cp
         out["final_cost_mean"] = float(np.mean([r.final_cost for r in reps]))
         s.close()
         return out
-    dev_s, wall_s = timed_solves(s, probs, iters, steps, warmup)
+    dev_s, wall_s, _ = timed_solves(s, probs, iters, steps, warmup)
     out["value"] = len(probs) * iters * steps / dev_s
     out["ms_per_step"] = dev_s / steps * 1e3
     reset_state(s, probs)
@@ -518,8 +550,10 @@ def run_ours(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    t_dev, wall = timed_solves(solver, probs, iters, args.steps, args.warmup, barrier, barrier if swarm else None)
+    t_dev, wall, last_reps = timed_solves(solver, probs, iters, args.steps, args.warmup, barrier, barrier if swarm else None)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, solver.get_blocks, probs, last_reps, f"_rank{rank}" if world > 1 else "")
     tt = torch.tensor([wall, t_dev], dtype=torch.float64, device="cuda")
     if dist is not None:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -702,7 +736,10 @@ def main():
     ap.add_argument("--host-threads", type=int, default=0, help="feeding / planning threads per stage of the e2e leg (0 = min(cores, 32))")
     ap.add_argument("--no-extras", action="store_true", help="N=1: skip the latency_b1 / swarm_1gpu legs")
     ap.add_argument("--impl", default="ours")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's solved state and costs as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     # watchdog: a rank stuck in a collective must not hang the launcher -- dump every thread's Python stack and exit
     import faulthandler
